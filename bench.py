@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the hot path: yolo26-master-n detection forward, synthetic 640x640 batches (BASELINE.json configs[1]).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 One "step" = one forward pass of a batch of 32 synthetic images per GPU (weak scaling: per-GPU batch fixed).
   value     images/s with the batch already resident in HBM (CUDA-graph replay of the whole forward, CUDA events,
@@ -100,6 +100,14 @@ class ClockSampler:
         return out
 
 
+def dump_outputs(out_dir, arrays):
+    """Writes each tensor as `out_dir/<name>.npy` (float32), so that the outputs of two builds on the same seeded inputs can be compared."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.detach().float().cpu().numpy())
+
+
 def pick_cpu_threads(forward_one):
     """The reference's PyTorch-CPU path does not scale to every core of a large host (N x N attention is memory bound):
     probe 8/16/32/64/all threads on one image and keep the fastest, so the CPU arm is shown at its best."""
@@ -164,8 +172,10 @@ def run_reference(args):
             fwd(xs[i % 2])
         t0 = time.perf_counter()
         for i in range(args.steps):
-            fwd(xs[i % 2])
+            y = fwd(xs[i % 2])
         dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"detections": y})
     v = B * args.steps / dt
     src = ("unmodified reference: oracle/_ref/ultralytics DetectionModel('yolo26-master-n.yaml').eval().fuse()" if kind == "reference"
            else "oracle port of the reference forward (oracle/_ref missing)")
@@ -517,6 +527,10 @@ def run_ours(args):
         ms_single = timed(lambda i: g(dev_in[i % nrot]), args.steps, args.warmup)
         ms_dev = timed_pipe(args.steps, args.warmup) if depth > 1 else ms_single
     clocks = clk.summary()
+    if args.dump_outputs and rank == 0:
+        # the headline path's last step: batch steps - 1 ran on pipeline instance (steps - 1) % depth (or on the single graph)
+        last = pipe.graphs[(args.steps - 1) % depth].static_out if depth > 1 else g.static_out
+        dump_outputs(args.dump_outputs, {"detections": last})
     # e2e: K batches through the public pipelined host-buffer API; every step's H2D (uint8 frames) and D2H ((B,300,6) fp32)
     # are inside the timed region, on copy streams that overlap the neighbouring steps' compute
     def e2e_run(n):
@@ -621,7 +635,11 @@ def main():
                     help="launch priority (0 = off, -1 .. -8) of every kernel except the attention kernels (ym_set_kernel_priority)")
     ap.add_argument("--depth-sweep", action="store_true", help="also time PipelinedForward at depth 1 / 2 / 3 / 4")
     ap.add_argument("--streams", type=int, default=4, help="graph instances / streams of PipelinedForward (1 = a single graph)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the (B, 300, 6) detections of the last timed step to DIR/detections.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
     # stdout carries exactly ONE JSON line: libraries that print to the C-level stdout (NCCL prints "NCCL version ..." there on
     # init) are redirected to stderr for the duration of the run; the JSON goes to the saved descriptor.

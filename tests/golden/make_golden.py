@@ -367,6 +367,39 @@ def letterbox_golden():
     torch.save({"cv2": cv2.__version__, "cases": cases, "variants": variants, "scale_boxes": boxes}, f"{OUT}/letterbox.golden.pt")
 
 
+def scale_coords_golden():
+    """The reference's `ops.scale_coords` (640x640 -> frame, with and without `normalize`) on seeded keypoints that straddle the
+    frame: inputs and fp32 outputs."""
+    from ultralytics.utils import ops
+    g = torch.Generator().manual_seed(12)
+    cases = []
+    for shape0 in ((480, 640), (1080, 1920), (100, 37), (640, 640)):
+        for norm in (False, True):
+            k = torch.rand((7, 17, 3), generator=g) * 800 - 60
+            cases.append({"shape0": shape0, "normalize": norm, "coords": k,
+                          "out": ops.scale_coords((640, 640), k.clone(), shape0, normalize=norm)})
+    torch.save({"cases": cases}, f"{OUT}/scale_coords.golden.pt")
+    print("scale_coords", len(cases), os.path.getsize(f"{OUT}/scale_coords.golden.pt"))
+
+
+def zoo_golden():
+    """The reference's model zoo as tests/test_zoo_builds.py reads it: every detection YAML (`master/**/det`, `master/exp`, the
+    `26/*master*` files) and the n file of every seg / pose / obb / cls family, parsed, keyed by the path below `cfg/models`, one
+    file per line."""
+    import glob
+
+    import ultralytics
+    import yaml
+    ref = os.path.join(os.path.dirname(ultralytics.__file__), "cfg", "models")
+    files = sorted(glob.glob(f"{ref}/master/**/*.yaml", recursive=True) + glob.glob(f"{ref}/26/*master*.yaml"))
+    files = [f for f in files if "/det/" in f or "/26/" in f or "/exp/" in f
+             or (any(f"/{t}/" in f for t in ("seg", "pose", "obb", "cls")) and f.endswith("-n.yaml"))]
+    rows = [f"{json.dumps(os.path.relpath(f, ref))}: {json.dumps(yaml.safe_load(open(f)), separators=(',', ':'))}" for f in files]
+    with open(f"{OUT}/zoo.golden.json", "w") as f:
+        f.write("{\n" + ",\n".join(rows) + "\n}\n")
+    print("zoo", len(rows), os.path.getsize(f"{OUT}/zoo.golden.json"))
+
+
 def cls_golden():
     """Reference ClassificationModel (v0_1 cls n: ModularRouterExpertMoE backbone + Classify) on seeded 64x64 images: probabilities,
     logits and the layer-11 feature; key table + calibrated BatchNorm statistics like the other model fixtures."""
@@ -454,10 +487,11 @@ def gated_family_golden():
 
 
 if __name__ == "__main__":
-    which = sys.argv[1:] or ["main", "dispatch", "nms", "postproc", "esmoe", "letterbox", "gated_family", "cls", *EXTRA_MODELS]
+    which = sys.argv[1:] or ["main", "dispatch", "nms", "postproc", "esmoe", "letterbox", "scale_coords", "zoo", "gated_family", "cls",
+                             *EXTRA_MODELS]
     for w in which:
         if w in EXTRA_MODELS:
             extra_model_golden(w)
         else:
             {"main": main, "dispatch": dispatch_golden, "nms": nms_golden, "postproc": postproc_golden, "esmoe": esmoe_golden, "letterbox": letterbox_golden,
-             "gated_family": gated_family_golden, "cls": cls_golden}[w]()
+             "gated_family": gated_family_golden, "cls": cls_golden, "scale_coords": scale_coords_golden, "zoo": zoo_golden}[w]()

@@ -68,27 +68,10 @@ def test_scale_boxes_oracle_matches_reference(case):
     assert np.array_equal(out, case["out"].numpy())
 
 
-def test_scale_coords_oracle_matches_reference(tmp_path):
-    """oracle scale_coords == the reference's ops.scale_coords, bit for bit (needs /root/reference: build container only).  The
-    reference runs in a subprocess, so that this process never imports ultralytics."""
-    import os
-    import subprocess
-    import sys
-    import numpy as np
-    import pytest
-    import torch
-    if not os.path.isdir("/root/reference/ultralytics"):
-        pytest.skip("reference tree not present")
-    from oracle import letterbox_oracle as L
-    g = torch.Generator().manual_seed(12)
-    cases = [(shape0, norm, torch.rand((7, 17, 3), generator=g) * 800 - 60)
-             for shape0 in ((480, 640), (1080, 1920), (100, 37), (640, 640)) for norm in (False, True)]
-    torch.save(cases, tmp_path / "cases.pt")
-    code = ("import sys, torch; sys.path.insert(0, '/root/reference'); from ultralytics.utils import ops as R; "
-            f"cases = torch.load('{tmp_path}/cases.pt'); "
-            "torch.save([R.scale_coords((640, 640), k.clone(), s, normalize=n) for s, n, k in cases], "
-            f"'{tmp_path}/want.pt')")
-    subprocess.run([sys.executable, "-c", code], check=True, env={**os.environ, "YOLO_CONFIG_DIR": "/tmp/ulcfg"}, capture_output=True)
-    want = torch.load(tmp_path / "want.pt")
-    for (shape0, norm, k), w in zip(cases, want):
-        assert np.array_equal(L.scale_coords((640, 640), k.numpy(), shape0, normalize=norm), w.numpy()), (shape0, norm)
+def test_scale_coords_oracle_matches_reference():
+    """oracle scale_coords == the reference's ops.scale_coords, bit for bit (fixture: tests/golden/make_golden.py scale_coords)."""
+    cases = torch.load(os.path.join(GOLD, "scale_coords.golden.pt"))["cases"]
+    assert len(cases) == 8
+    for c in cases:
+        out = L.scale_coords((640, 640), c["coords"].numpy(), c["shape0"], normalize=c["normalize"])
+        assert np.array_equal(out, c["out"].numpy()), (c["shape0"], c["normalize"])
